@@ -79,16 +79,17 @@ SYMBOLS = {
 _lib = None
 
 
-def load():
-    """dlopen libgsplat_b200.so and type every entry point.  Raises if the library was not built."""
+def load(path: str = LIB_PATH):
+    """dlopen libgsplat_b200.so (the in-tree build unless `path` names another) and type every entry point.  Raises if
+    the library was not built.  The first call decides which library the process uses."""
     global _lib
     if _lib is not None:
         return _lib
-    if not os.path.exists(LIB_PATH):
+    if not os.path.exists(path):
         raise RuntimeError(
-            f"{LIB_PATH} is missing: build it with __graft_entry__.build() "
+            f"{path} is missing: build it with __graft_entry__.build() "
             "(nvcc, sm_100a).  There is no CPU fallback for the splat path.")
-    lib = C.CDLL(LIB_PATH)
+    lib = C.CDLL(path)
     for name, (res, args) in SYMBOLS.items():
         fn = getattr(lib, name)  # AttributeError if the header and the library disagree
         fn.restype = res

@@ -21,27 +21,27 @@ NVCC_FLAGS = [
 ]
 
 
-def _stale() -> bool:
-    if not os.path.exists(LIB):
+def stale(out: str = LIB) -> bool:
+    if not os.path.exists(out):
         return True
-    t = os.path.getmtime(LIB)
+    t = os.path.getmtime(out)
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", "gsplat_b200.h")]
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_library(force: bool = False, verbose: bool = False) -> str:
-    """Compile libgsplat_b200.so next to this file (cross-compiles without a GPU)."""
-    if not force and not _stale():
-        return LIB
+def build_library(force: bool = False, verbose: bool = False, out: str = LIB) -> str:
+    """Compile libgsplat_b200.so to `out`, by default next to this file (cross-compiles without a GPU)."""
+    if not force and not stale(out):
+        return out
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
     extra = os.environ.get("GS_NVCC_EXTRA", "").split()
-    cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + [os.path.join(CSRC, s) for s in SOURCES]
+    cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", out] + [os.path.join(CSRC, s) for s in SOURCES]
     res = subprocess.run(cmd, capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + res.stdout + res.stderr)
     if verbose:
         sys.stderr.write(res.stderr)
-    return LIB
+    return out
 
 
 if __name__ == "__main__":

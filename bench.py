@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle restatement)
+    python bench.py ... --dump-outputs DIR                   # also save the frame of the last timed step (frame_outputs)
 
 A "step" is one full frame of the workload: the worker sort request plus the instanced draw
 (reference index.js:438-455 + 184-207), synchronously with the same camera.
@@ -46,6 +47,44 @@ METRICS = {
 }
 FRAME_TOL = 1e-3
 DTYPE = "f64 sort keys + f32 shading"
+DUMP_BYTES = 64_000_000  # --dump-outputs: total size of the .npy files
+
+
+def load_gsplat(gs):
+    """The CUDA library as build() left it in the tree.  One that is missing or older than its sources is compiled into
+    a temporary directory instead: the bench writes nothing into the tree, which may be read-only."""
+    if not gs.build.stale():
+        return gs._lib.load()
+    with tempfile.TemporaryDirectory(prefix="gsplat_bench_") as tmp:
+        return gs._lib.load(gs.build.build_library(out=os.path.join(tmp, "libgsplat_b200.so")))
+
+
+def load_oracle():
+    """The CPU oracle, found or compiled like the CUDA library in load_gsplat()."""
+    from oracle import oracle as orc
+    if orc.stale():
+        with tempfile.TemporaryDirectory(prefix="gsplat_bench_") as tmp:
+            orc.lib(orc.build(out=os.path.join(tmp, "libgs_oracle.so")))
+    return orc
+
+
+def frame_outputs(frame: np.ndarray) -> dict:
+    """--dump-outputs arrays of one (H, W, 4) RGBA8 frame (row 0 = bottom), as float32 byte values: `frame` when the
+    whole frame fits DUMP_BYTES, otherwise a fixed seeded sample of its pixels, `frame_pixels` (k, 4), and their
+    row-major pixel indices, `frame_pixel_index` (k,) float64.  Same frame -> same arrays."""
+    f = np.ascontiguousarray(frame, np.float32)
+    if f.nbytes <= DUMP_BYTES - 4096:  # room for the .npy headers
+        return {"frame": f}
+    px = f.reshape(-1, f.shape[-1])
+    k = (DUMP_BYTES - 4096) // (px.itemsize * px.shape[1] + 8)
+    idx = np.sort(np.random.default_rng(0).choice(px.shape[0], k, replace=False))
+    return {"frame_pixels": px[idx], "frame_pixel_index": idx.astype(np.float64)}
+
+
+def write_outputs(out_dir: str, arrays: dict) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -198,8 +237,7 @@ def run_reference(args):
     if rank != 0:
         return
     gs = importlib.import_module("aframe-gaussian-splatting_b200")
-    from oracle import oracle as orc
-    orc.build()
+    orc = load_oracle()
     rows, frames, n, w, h = build_scene(gs, args.workload, args.splats)
     threads = cpu_threads(orc)
     cs, cc, m = orc.pack(rows)
@@ -314,7 +352,7 @@ def run_ours(args):
         dist.init_process_group("nccl", rank=rank, world_size=world, device_id=torch.device("cuda", local), pg_options=opts)
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    gs.build.build_library()
+    load_gsplat(gs)
     ctx = gs.SplatContext(local)
     stream = torch.cuda.ExternalStream(ctx._lib.gs_stream(ctx._h), device=dev)
     with torch.cuda.stream(stream):
@@ -324,6 +362,7 @@ def run_ours(args):
     uuid = str(torch.cuda.get_device_properties(dev).uuid)
     uuid = uuid if uuid.startswith("GPU-") else "GPU-" + uuid
     peak, peak_src = load_peaks()
+    dump = {}  # --dump-outputs arrays of the headline configuration
 
     def barrier():
         if world > 1:
@@ -404,12 +443,12 @@ def run_ours(args):
             ctx.assemble_tiles(gath_bufs[i % 3].data_ptr(), tiles_per_rank, world, w, h, gs.GS_FORMAT_RGBA8, frames_dev[i % 3].data_ptr())
             return t
 
-        def run_pipeline(submit, k, collect=None, depth=3):
+        def run_pipeline(submit, k, collect=None, depth=3, tickets=None):
             """k frames, at most `depth` outstanding (3: sort(i) | bin(i-1) | raster(i-2); 4 when frames also cross PCIe:
             + copy(i-3)); one CUDA-event pair on the library's stream brackets everything (the L2 flushes between steps
-            included)."""
+            included).  The frames' tickets are appended to `tickets` when a list is given."""
             r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            tickets = []
+            tickets = [] if tickets is None else tickets
             with torch.cuda.stream(stream):
                 r0.record(stream)
             for i in range(k):
@@ -441,7 +480,14 @@ def run_ours(args):
 
         # ---- value: device-resident frames ----
         barrier()
-        my_ms = run_pipeline(submit_device, steps, depth=3 if sharded else args.value_depth)
+        timed = []
+        my_ms = run_pipeline(submit_device, steps, depth=3 if sharded else args.value_depth, tickets=timed)
+        if headline and rank == 0 and args.dump_outputs:
+            # the frame of the last timed step, read before the untimed frames below reuse its buffer
+            last = np.empty((h, w, 4), np.uint8)
+            src = ctx.peer_frame(timed[-1]) if use_peer else frames_dev[(steps - 1) % (3 if sharded else 4)].data_ptr()
+            ctx.memcpy_d2h(last, src, last.nbytes)
+            dump.update(frame_outputs(last))
         total_ms = allmax(my_ms)
         barrier()
         if world > 1:
@@ -589,8 +635,7 @@ def run_ours(args):
             if frame_check is not None:
                 res["frame_check"] = frame_check
             if world == 1 and not args.no_cpu_baseline:
-                from oracle import oracle as orc
-                orc.build()
+                orc = load_oracle()
                 threads = cpu_threads(orc)
                 par, cpu = parity_block(gs, orc, ctx, rows, frames[40 % nf], w, h, threads)
                 res["parity"] = par
@@ -633,6 +678,8 @@ def run_ours(args):
         if alt is not None:
             line["alt_parallel"] = alt
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dump)
         bad = [x for x in [head] + others if isinstance(x.get("parity"), dict) and not x["parity"]["ok"]]
         if bad:
             sys.stderr.write("[bench] PARITY FAILURE: " + ", ".join(f"{x['config']['workload']} max_abs_err={x['parity']['max_abs_err']:.3g}" for x in bad) + "\n")
@@ -663,7 +710,14 @@ def main():
                          "`tiles` = one frame sharded by screen bin columns + tile exchange (strong scaling, default for the 80 M scene)")
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"],
                     help="multi-GPU frame exchange: fused raster + NVLink peer stores (default) or NCCL all-gather of tiles")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the RGBA8 frame of the last timed step of the headline configuration (as float32) to "
+                         "DIR/<name>.npy, at most 64 MB: a seeded sample of the pixels when the frame is larger")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm shades only a band of rows per step; use it with --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

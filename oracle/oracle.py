@@ -15,13 +15,17 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libgs_oracle.so")
 
 
-def build(force: bool = False) -> str:
-    src = os.path.join(HERE, "gs_oracle.c")
-    if force or not os.path.exists(LIB_PATH) or os.path.getmtime(LIB_PATH) < os.path.getmtime(src):
-        res = subprocess.run(["make", "-C", HERE, "-B" if force else "-s"], capture_output=True, text=True)
+def stale(out: str = LIB_PATH) -> bool:
+    return not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(os.path.join(HERE, "gs_oracle.c"))
+
+
+def build(force: bool = False, out: str = LIB_PATH) -> str:
+    """Compile libgs_oracle.so to `out`, by default next to this file."""
+    if force or stale(out):
+        res = subprocess.run(["make", "-C", HERE, "-B" if force else "-s", f"OUT={os.path.abspath(out)}"], capture_output=True, text=True)
         if res.returncode != 0:
             raise RuntimeError("oracle build failed:\n" + res.stdout + res.stderr)
-    return LIB_PATH
+    return out
 
 
 class ProjRec(C.Structure):
@@ -38,11 +42,11 @@ class RenderStats(C.Structure):
 _lib = None
 
 
-def lib():
+def lib(path: str | None = None):
+    """The loaded oracle library: `path`, or the in-tree build (compiled first when stale).  The first call decides."""
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(LIB_PATH)
+        L = C.CDLL(build() if path is None else path)
         L.orc_pack.restype = C.c_int
         L.orc_sort.restype = C.c_int
         L.orc_sort_compact.restype = C.c_int

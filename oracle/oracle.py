@@ -39,6 +39,10 @@ class RenderStats(C.Structure):
     _fields_ = [("n_order", C.c_uint32), ("n_visible", C.c_uint32), ("fragments", C.c_uint64)]
 
 
+class F2bStats(C.Structure):
+    _fields_ = [("hits_eager", C.c_uint64), ("hits_lazy", C.c_uint64), ("n_differ", C.c_uint64), ("max_m", C.c_double)]
+
+
 _lib = None
 
 
@@ -54,6 +58,7 @@ def lib(path: str | None = None):
         L.orc_render.restype = C.c_int
         L.orc_render_rows.restype = C.c_int
         L.orc_render_ex.restype = C.c_int
+        L.orc_render_f2b.restype = C.c_int
         L.orc_coverage_check.restype = C.c_int
         L.orc_set_affinity.restype = None
         L.orc_ply_to_splat.restype = C.c_int64
@@ -184,6 +189,29 @@ def render(center_scale, cov_color, order, proj, mv, width, height, focal, bg=(0
                              C.c_uint32(r0), C.c_uint32(r1), _p(d))
     assert rc == 0
     return out, {"n_order": st.n_order, "n_visible": st.n_visible, "fragments": st.fragments}
+
+
+def render_f2b(center_scale, cov_color, order, proj, mv, width, height, focal, t_stop=3e-4, exact=False, depth_in=None,
+               nthreads=None):
+    """Front-to-back fp64 reference of the CUDA raster with its stop rule bracketed (orc_render_f2b in gs_oracle.c).
+    Returns (eager, lazy, stats): two (H, W, 4) float64 frames {R, G, B, T} (row 0 = bottom, no background) and
+    {"hits_eager", "hits_lazy", "n_differ", "max_m"}.  t_stop=0 disables the stop; exact=True applies the stop rule to
+    the fp64 transmittance without an error margin (then eager == lazy)."""
+    cs = np.ascontiguousarray(center_scale, np.float32).reshape(-1, 4)
+    cc = np.ascontiguousarray(cov_color, np.uint32).reshape(-1, 4)
+    o = np.ascontiguousarray(order, np.uint32)
+    eager = np.zeros((height, width, 4), np.float64)
+    lazy = np.zeros((height, width, 4), np.float64)
+    st = F2bStats()
+    if nthreads is None:
+        nthreads = os.cpu_count() or 1
+    d = None if depth_in is None else np.ascontiguousarray(depth_in, np.float32).reshape(height, width)
+    rc = lib().orc_render_f2b(_p(cs), _p(cc), _p(o), C.c_uint32(o.shape[0]), _p(np.ascontiguousarray(proj, np.float32)),
+                              _p(np.ascontiguousarray(mv, np.float32)), C.c_uint32(width), C.c_uint32(height), C.c_float(focal),
+                              _p(d), C.c_double(t_stop), C.c_int(1 if exact else 0), _p(eager), _p(lazy), C.byref(st),
+                              C.c_int(nthreads))
+    assert rc == 0
+    return eager, lazy, {"hits_eager": st.hits_eager, "hits_lazy": st.hits_lazy, "n_differ": st.n_differ, "max_m": st.max_m}
 
 
 def coverage_check(center_scale, cov_color, order, proj, mv, width, height, focal, nthreads=None) -> dict:

@@ -123,6 +123,9 @@ def test_stats_frame_counts(gs, orc, ctx):
     assert st["n_records_streamed"] >= st["n_tile_instances"]
     assert 0 < st["n_pair_hits"] <= st["n_pair_tests"]
     assert st["n_pair_hits"] <= pairs * 1.001 + 16                     # early-stopped pixels skip pairs, never add any
+    # exact: every covered pair at a live pixel is blended; the front-to-back reference brackets where pixels stop
+    _, _, f2b = orc.render_f2b(cs, cc, order, fr.proj, fr.modelview, w, h, fr.focal)
+    assert f2b["hits_eager"] <= st["n_pair_hits"] <= f2b["hits_lazy"]
 
 
 def _eye_cameras(gs, w, h, ipd=0.064):

@@ -169,9 +169,10 @@ def test_render_parity(gs, orc, ctx, n, w, h, cutout, fmt):
         assert d.max() <= 2 and (d <= 1).mean() >= 0.999
         assert (d == 0).mean() > 0.98
     st = ctx.stats()
-    assert st["n_sorted"] == len(order) and st["n_visible"] >= est["n_visible"] * 0 and st["n_instances"] > 0
+    assert st["n_sorted"] == len(order) and st["n_instances"] > 0
     assert st["width"] == w and st["height"] == h and st["n_tiles"] == ((w + 15) // 16) * ((h + 15) // 16)
-    _check_projection(gs, orc, ctx, cs, cc, fr, order)
+    # V2 counts the draw-order entries with a bin rectangle: the splats the GPU binned, no more than the oracle's visible
+    assert st["n_dropped"] == 0 and st["n_visible"] == _check_projection(gs, orc, ctx, cs, cc, fr, order) <= est["n_visible"]
 
 
 def test_render_golden(gs, orc, ctx):
